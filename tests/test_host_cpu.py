@@ -101,10 +101,9 @@ def test_reference_checkpoint_loads_strictly(golden_dir):
         net.load_state_dict(sd, strict=True)
 
 
-def test_yaml_configs_drop_in():
-    ref_cfgs = os.environ.get("SGB_REFERENCE_CONFIGS", "/root/reference/src/configs")
-    if not os.path.isdir(ref_cfgs):
-        pytest.skip("reference config tree not present on this box")
+def test_yaml_configs_drop_in(golden_dir):
+    # unmodified copies of the reference's src/configs files
+    ref_cfgs = os.path.join(golden_dir, "reference_configs")
     for rel in ["ImageNet/BigGAN-Deep-256.yaml", "CIFAR10/BigGAN.yaml", "CIFAR10/SNGAN.yaml", "CIFAR10/WGAN-GP.yaml",
                 "CIFAR10/BigGAN-Deep.yaml"]:
         cfg = C.Configurations(os.path.join(ref_cfgs, rel))
