@@ -61,119 +61,60 @@ __device__ __forceinline__ uint32_t pack_bf16x2(float a, float b) {
   return *reinterpret_cast<uint32_t*>(&t);
 }
 
-__device__ __forceinline__ bool epi_vec_ok(const EpiArgs& p) {
+// Operand alignment of the vector epilogue paths: whole 8-channel units, 16-byte aligned rows of every bf16 operand.
+__host__ __device__ inline bool epi_vec_ok(const EpiArgs& p) {
   return (p.Cout % 8 == 0) && (p.y_cstride % 8 == 0) && (p.residual == nullptr || p.res_cstride % 8 == 0) &&
          (p.mask == nullptr || p.mask_cstride % 8 == 0);
 }
+// A launch can stage its output tile in shared memory and write it with TMA tensor stores: bf16 output, whole 64-channel
+// chunks per tile, aligned operands.
+__host__ __device__ inline bool epi_can_stage(const EpiArgs& p, int BN) {
+  return !p.y_fp32 && (BN % 64 == 0) && epi_vec_ok(p);
+}
 
-// One thread = one accumulator row (TMEM lane).  t_row: TMEM address of this warp's lane quadrant at the accumulator's
-// first column.  All 32 lanes of the warp must call this (tcgen05.ld is warp-collective); stores are predicated by valid.
-__device__ __forceinline__ void epilogue_row(const EpiArgs& p, uint32_t t_row, int BN, int n0, bool valid, long long pix,
-                                             long long rpix, float alpha, bool vec_ok) {
-  const bool res_pre = p.residual != nullptr && !p.res_after;
-  const bool res_post = p.residual != nullptr && p.res_after;
-  const float rs = p.res_scale;
-  for (int c0 = 0; c0 < BN; c0 += 16) {
-    uint32_t v[16];
-    __syncwarp();
-    tmem_ld16(t_row + c0, v);
-    tmem_ld_wait();
-    const int n = n0 + c0;
-    if (!valid || n >= p.Cout) continue;
-    float f[16];
+// One 16-column piece of the epilogue.  Every store path runs the same steps in the same order (alpha, [softmax], bias,
+// residual, ReLU, mask, post-mask residual, pack), so their outputs are bit-identical; where a bf16 operand comes from (the
+// aux ring in shared memory, __ldg, or zeros past a ragged channel tail) is the caller's choice.
+__device__ __forceinline__ void piece_bias(float (&f)[16], const float* bias, int nvalid) {
+  const float4* bp = reinterpret_cast<const float4*>(bias);
 #pragma unroll
-    for (int j = 0; j < 16; ++j) f[j] = __uint_as_float(v[j]) * alpha;
-    if (vec_ok && n + 16 <= p.Cout) {
-      if (p.bias) {
-        const float4* bp = reinterpret_cast<const float4*>(p.bias + n);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const float4 bb = __ldg(bp + j);
-          f[4 * j + 0] += bb.x; f[4 * j + 1] += bb.y; f[4 * j + 2] += bb.z; f[4 * j + 3] += bb.w;
-        }
-      }
-      if (res_pre) {
-        const uint4* rp = reinterpret_cast<const uint4*>(p.residual + rpix * p.res_cstride + n);
-#pragma unroll
-        for (int j = 0; j < 2; ++j) {
-          const uint4 r = __ldg(rp + j);
-          f[8 * j + 0] = fmaf(bf16_bits_lo(r.x), rs, f[8 * j + 0]); f[8 * j + 1] = fmaf(bf16_bits_hi(r.x), rs, f[8 * j + 1]);
-          f[8 * j + 2] = fmaf(bf16_bits_lo(r.y), rs, f[8 * j + 2]); f[8 * j + 3] = fmaf(bf16_bits_hi(r.y), rs, f[8 * j + 3]);
-          f[8 * j + 4] = fmaf(bf16_bits_lo(r.z), rs, f[8 * j + 4]); f[8 * j + 5] = fmaf(bf16_bits_hi(r.z), rs, f[8 * j + 5]);
-          f[8 * j + 6] = fmaf(bf16_bits_lo(r.w), rs, f[8 * j + 6]); f[8 * j + 7] = fmaf(bf16_bits_hi(r.w), rs, f[8 * j + 7]);
-        }
-      }
-      if (p.relu) {
-#pragma unroll
-        for (int j = 0; j < 16; ++j) f[j] = fmaxf(f[j], 0.f);
-        if (p.relu_bits)
-          reinterpret_cast<unsigned short*>(p.relu_bits)[(pix * (p.Cout >> 6) + (n >> 6)) * 4 + ((n >> 4) & 3)] =
-              (unsigned short)positive_bits16(f);
-      }
-      if (p.mask_bits) {
-        apply_bits16(f, __ldg(reinterpret_cast<const unsigned short*>(p.mask_bits) + (pix * (p.Cout >> 6) + (n >> 6)) * 4 + ((n >> 4) & 3)));
-      } else if (p.mask) {
-        const uint4* mp = reinterpret_cast<const uint4*>(p.mask + pix * p.mask_cstride + n);
-#pragma unroll
-        for (int j = 0; j < 2; ++j) {
-          const uint4 m = __ldg(mp + j);
-          f[8 * j + 0] = bf16_bits_lo(m.x) > 0.f ? f[8 * j + 0] : 0.f;
-          f[8 * j + 1] = bf16_bits_hi(m.x) > 0.f ? f[8 * j + 1] : 0.f;
-          f[8 * j + 2] = bf16_bits_lo(m.y) > 0.f ? f[8 * j + 2] : 0.f;
-          f[8 * j + 3] = bf16_bits_hi(m.y) > 0.f ? f[8 * j + 3] : 0.f;
-          f[8 * j + 4] = bf16_bits_lo(m.z) > 0.f ? f[8 * j + 4] : 0.f;
-          f[8 * j + 5] = bf16_bits_hi(m.z) > 0.f ? f[8 * j + 5] : 0.f;
-          f[8 * j + 6] = bf16_bits_lo(m.w) > 0.f ? f[8 * j + 6] : 0.f;
-          f[8 * j + 7] = bf16_bits_hi(m.w) > 0.f ? f[8 * j + 7] : 0.f;
-        }
-      }
-      if (res_post) {
-        const uint4* rp = reinterpret_cast<const uint4*>(p.residual + rpix * p.res_cstride + n);
-#pragma unroll
-        for (int j = 0; j < 2; ++j) {
-          const uint4 r = __ldg(rp + j);
-          f[8 * j + 0] = fmaf(bf16_bits_lo(r.x), rs, f[8 * j + 0]); f[8 * j + 1] = fmaf(bf16_bits_hi(r.x), rs, f[8 * j + 1]);
-          f[8 * j + 2] = fmaf(bf16_bits_lo(r.y), rs, f[8 * j + 2]); f[8 * j + 3] = fmaf(bf16_bits_hi(r.y), rs, f[8 * j + 3]);
-          f[8 * j + 4] = fmaf(bf16_bits_lo(r.z), rs, f[8 * j + 4]); f[8 * j + 5] = fmaf(bf16_bits_hi(r.z), rs, f[8 * j + 5]);
-          f[8 * j + 6] = fmaf(bf16_bits_lo(r.w), rs, f[8 * j + 6]); f[8 * j + 7] = fmaf(bf16_bits_hi(r.w), rs, f[8 * j + 7]);
-        }
-      }
-      if (p.y_fp32) {
-        float4* yp = reinterpret_cast<float4*>(reinterpret_cast<float*>(p.y) + pix * p.y_cstride + n);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) yp[j] = make_float4(f[4 * j], f[4 * j + 1], f[4 * j + 2], f[4 * j + 3]);
-      } else {
-        uint4* yp = reinterpret_cast<uint4*>(reinterpret_cast<bf16*>(p.y) + pix * p.y_cstride + n);
-#pragma unroll
-        for (int j = 0; j < 2; ++j) {
-          uint4 o;
-          o.x = pack_bf16x2(f[8 * j + 0], f[8 * j + 1]);
-          o.y = pack_bf16x2(f[8 * j + 2], f[8 * j + 3]);
-          o.z = pack_bf16x2(f[8 * j + 4], f[8 * j + 5]);
-          o.w = pack_bf16x2(f[8 * j + 6], f[8 * j + 7]);
-          yp[j] = o;
-        }
-      }
-    } else {
-      // ragged / unaligned channel tail (e.g. Cout = 3): scalar path
-#pragma unroll
-      for (int j = 0; j < 16; ++j) {
-        const int nn = n + j;
-        if (nn < p.Cout) {
-          float x = f[j];
-          if (p.bias) x += __ldg(p.bias + nn);
-          if (res_pre) x = fmaf(__bfloat162float(p.residual[rpix * p.res_cstride + nn]), rs, x);
-          if (p.relu) x = fmaxf(x, 0.f);
-          if (p.mask) x = __bfloat162float(p.mask[pix * p.mask_cstride + nn]) > 0.f ? x : 0.f;
-          if (res_post) x = fmaf(__bfloat162float(p.residual[rpix * p.res_cstride + nn]), rs, x);
-          if (p.y_fp32) reinterpret_cast<float*>(p.y)[pix * p.y_cstride + nn] = x;
-          else reinterpret_cast<bf16*>(p.y)[pix * p.y_cstride + nn] = __float2bfloat16_rn(x);
-        }
-      }
+  for (int j = 0; j < 4; ++j) {
+    if (4 * j < nvalid) {
+      const float4 bb = __ldg(bp + j);
+      f[4 * j + 0] += bb.x; f[4 * j + 1] += bb.y; f[4 * j + 2] += bb.z; f[4 * j + 3] += bb.w;
     }
   }
 }
-
+// f += rs * r for the 16 bf16 values of two 16-byte units
+__device__ __forceinline__ void piece_res_fma(float (&f)[16], uint4 r0, uint4 r1, float rs) {
+#pragma unroll
+  for (int j = 0; j < 2; ++j) {
+    const uint4 r = j ? r1 : r0;
+    f[8 * j + 0] = fmaf(bf16_bits_lo(r.x), rs, f[8 * j + 0]); f[8 * j + 1] = fmaf(bf16_bits_hi(r.x), rs, f[8 * j + 1]);
+    f[8 * j + 2] = fmaf(bf16_bits_lo(r.y), rs, f[8 * j + 2]); f[8 * j + 3] = fmaf(bf16_bits_hi(r.y), rs, f[8 * j + 3]);
+    f[8 * j + 4] = fmaf(bf16_bits_lo(r.z), rs, f[8 * j + 4]); f[8 * j + 5] = fmaf(bf16_bits_hi(r.z), rs, f[8 * j + 5]);
+    f[8 * j + 6] = fmaf(bf16_bits_lo(r.w), rs, f[8 * j + 6]); f[8 * j + 7] = fmaf(bf16_bits_hi(r.w), rs, f[8 * j + 7]);
+  }
+}
+// f = (m > 0) ? f : 0 for the 16 bf16 mask values of two 16-byte units
+__device__ __forceinline__ void piece_mask_bf16(float (&f)[16], uint4 m0, uint4 m1) {
+#pragma unroll
+  for (int j = 0; j < 2; ++j) {
+    const uint4 m = j ? m1 : m0;
+    f[8 * j + 0] = bf16_bits_lo(m.x) > 0.f ? f[8 * j + 0] : 0.f;
+    f[8 * j + 1] = bf16_bits_hi(m.x) > 0.f ? f[8 * j + 1] : 0.f;
+    f[8 * j + 2] = bf16_bits_lo(m.y) > 0.f ? f[8 * j + 2] : 0.f;
+    f[8 * j + 3] = bf16_bits_hi(m.y) > 0.f ? f[8 * j + 3] : 0.f;
+    f[8 * j + 4] = bf16_bits_lo(m.z) > 0.f ? f[8 * j + 4] : 0.f;
+    f[8 * j + 5] = bf16_bits_hi(m.z) > 0.f ? f[8 * j + 5] : 0.f;
+    f[8 * j + 6] = bf16_bits_lo(m.w) > 0.f ? f[8 * j + 6] : 0.f;
+    f[8 * j + 7] = bf16_bits_hi(m.w) > 0.f ? f[8 * j + 7] : 0.f;
+  }
+}
+__device__ __forceinline__ void piece_pack(const float (&f)[16], uint32_t (&w)[8]) {
+#pragma unroll
+  for (int j = 0; j < 8; ++j) w[j] = pack_bf16x2(f[2 * j], f[2 * j + 1]);
+}
 
 // -------------------------------------------------------------------------------------------------------------------
 // Epilogue v2 (bf16 NHWC output, channel tile a multiple of 64): two teams of four warps take alternate 64-channel
@@ -202,10 +143,6 @@ __device__ __forceinline__ uint4 ld_shared_v4(uint32_t addr) {
   return r;
 }
 static constexpr int kEpiStageBytes = 128 * 128;  // one 128-row x 64-channel bf16 chunk
-
-__device__ __forceinline__ bool epi_use_tma(const EpiArgs& p, int BN) {
-  return !p.y_fp32 && (BN % 64 == 0) && epi_vec_ok(p);
-}
 
 // Compile-time epilogue variants.  The per-piece loop below runs on 2 warps per scheduler with little latency hiding, so
 // every run-time test of "is there a bias / residual / mask / ragged channel tail" costs issue slots on the critical path of
@@ -281,107 +218,104 @@ __device__ __forceinline__ void epilogue_tile_smstats(const EpiArgs& p, uint32_t
   }
 }
 
-// Direct-store epilogue of a compile-time variant F >= 0 (bf16 output, Cout % 64 == 0, 16-byte aligned operands): the same
-// arithmetic as epilogue_row without its run-time case analysis, two 16-column pieces per TMEM wait.  Used by the halo-row
+// Direct-store epilogue.  One thread = one accumulator row (TMEM lane); t_row: TMEM address of this warp's lane quadrant at
+// the accumulator's first column.  All 32 lanes of the warp must call this (tcgen05.ld is warp-collective); stores are
+// predicated by valid.  F < 0: run-time flags, bf16 or fp32 output, scalar path for a ragged / unaligned channel tail.
+// F >= 0 (bf16 output, Cout % 64 == 0, 16-byte aligned operands): two 16-column pieces per TMEM wait.  Used by the halo-row
 // kernel's second output row at C = 64 (no room for a second staging tile): one full 128-byte line per thread and piece pair.
 template <int F>
-__device__ __forceinline__ void epilogue_row_fast(const EpiArgs& p, uint32_t t_row, int BN, int n0, bool valid, long long pix,
-                                                  long long rpix, float alpha) {
-  static_assert(F >= 0 && (F & kEpiFull), "compile-time variant with a full channel tile");
-  constexpr bool has_bias = (F & kEpiBias) != 0, do_relu = (F & kEpiRelu) != 0, res_pre = (F & kEpiResPre) != 0,
-                 res_post = (F & kEpiResPost) != 0, has_mask = (F & kEpiMask) != 0;
+__device__ __forceinline__ void epilogue_row(const EpiArgs& p, uint32_t t_row, int BN, int n0, bool valid, long long pix,
+                                             long long rpix, float alpha, bool vec_ok) {
+  static_assert(F < 0 || (F & kEpiFull), "compile-time variants have a full channel tile");
+  constexpr int NP = F >= 0 ? 2 : 1;
+  const bool has_bias = F < 0 ? p.bias != nullptr : (F & kEpiBias) != 0;
+  const bool do_relu = F < 0 ? p.relu != 0 : (F & kEpiRelu) != 0;
+  const bool res_pre = F < 0 ? (p.residual != nullptr && !p.res_after) : (F & kEpiResPre) != 0;
+  const bool res_post = F < 0 ? (p.residual != nullptr && p.res_after) : (F & kEpiResPost) != 0;
+  const bool use_mbits = F < 0 ? p.mask_bits != nullptr : (F & kEpiMaskBits) != 0;
+  const bool has_mask = F < 0 ? p.mask != nullptr : (F & kEpiMask) != 0;
+  const bool emit_bits = F < 0 ? p.relu_bits != nullptr : (F & kEpiBitsOut) != 0;
+  const bool y_fp32 = F < 0 && p.y_fp32;
   const float rs = p.res_scale;
-  bf16* yrow = reinterpret_cast<bf16*>(p.y) + pix * p.y_cstride;
-  for (int c0 = 0; c0 < BN; c0 += 32) {
-    uint32_t v[2][16];
+  for (int c0 = 0; c0 < BN; c0 += 16 * NP) {
+    uint32_t v[NP][16];
     __syncwarp();
-    tmem_ld16(t_row + c0, v[0]);
-    tmem_ld16(t_row + c0 + 16, v[1]);
+#pragma unroll
+    for (int q = 0; q < NP; ++q) tmem_ld16(t_row + c0 + 16 * q, v[q]);
     tmem_ld_wait();
     if (!valid || n0 + c0 >= p.Cout) continue;
 #pragma unroll
-    for (int q = 0; q < 2; ++q) {
-      const int n = n0 + c0 + q * 16;
+    for (int q = 0; q < NP; ++q) {
+      const int n = n0 + c0 + 16 * q;
       float f[16];
 #pragma unroll
       for (int j = 0; j < 16; ++j) f[j] = __uint_as_float(v[q][j]) * alpha;
-      if (has_bias) {
-        const float4* bp = reinterpret_cast<const float4*>(p.bias + n);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const float4 bb = __ldg(bp + j);
-          f[4 * j + 0] += bb.x; f[4 * j + 1] += bb.y; f[4 * j + 2] += bb.z; f[4 * j + 3] += bb.w;
-        }
-      }
-      if (res_pre || res_post) {
-        // (residual variants are not instantiated for this path today; kept for completeness of the flag set)
-        const uint4* rp = reinterpret_cast<const uint4*>(p.residual + rpix * p.res_cstride + n);
+      if (F >= 0 || (vec_ok && n + 16 <= p.Cout)) {
+        if (has_bias) piece_bias(f, p.bias + n, 16);
         if (res_pre) {
+          const uint4* rp = reinterpret_cast<const uint4*>(p.residual + rpix * p.res_cstride + n);
+          piece_res_fma(f, __ldg(rp), __ldg(rp + 1), rs);
+        }
+        if (do_relu) {
 #pragma unroll
-          for (int j = 0; j < 2; ++j) {
-            const uint4 r = __ldg(rp + j);
-            f[8 * j + 0] = fmaf(bf16_bits_lo(r.x), rs, f[8 * j + 0]); f[8 * j + 1] = fmaf(bf16_bits_hi(r.x), rs, f[8 * j + 1]);
-            f[8 * j + 2] = fmaf(bf16_bits_lo(r.y), rs, f[8 * j + 2]); f[8 * j + 3] = fmaf(bf16_bits_hi(r.y), rs, f[8 * j + 3]);
-            f[8 * j + 4] = fmaf(bf16_bits_lo(r.z), rs, f[8 * j + 4]); f[8 * j + 5] = fmaf(bf16_bits_hi(r.z), rs, f[8 * j + 5]);
-            f[8 * j + 6] = fmaf(bf16_bits_lo(r.w), rs, f[8 * j + 6]); f[8 * j + 7] = fmaf(bf16_bits_hi(r.w), rs, f[8 * j + 7]);
+          for (int j = 0; j < 16; ++j) f[j] = fmaxf(f[j], 0.f);
+          if (emit_bits)
+            reinterpret_cast<unsigned short*>(p.relu_bits)[(pix * (p.Cout >> 6) + (n >> 6)) * 4 + ((n >> 4) & 3)] =
+                (unsigned short)positive_bits16(f);
+        }
+        if (use_mbits) {
+          apply_bits16(f, __ldg(reinterpret_cast<const unsigned short*>(p.mask_bits) + (pix * (p.Cout >> 6) + (n >> 6)) * 4 + ((n >> 4) & 3)));
+        } else if (has_mask) {
+          const uint4* mp = reinterpret_cast<const uint4*>(p.mask + pix * p.mask_cstride + n);
+          piece_mask_bf16(f, __ldg(mp), __ldg(mp + 1));
+        }
+        if (res_post) {
+          const uint4* rp = reinterpret_cast<const uint4*>(p.residual + rpix * p.res_cstride + n);
+          piece_res_fma(f, __ldg(rp), __ldg(rp + 1), rs);
+        }
+        if (y_fp32) {
+          float4* yp = reinterpret_cast<float4*>(reinterpret_cast<float*>(p.y) + pix * p.y_cstride + n);
+#pragma unroll
+          for (int j = 0; j < 4; ++j) yp[j] = make_float4(f[4 * j], f[4 * j + 1], f[4 * j + 2], f[4 * j + 3]);
+        } else {
+          uint32_t w[8];
+          piece_pack(f, w);
+          uint4* yp = reinterpret_cast<uint4*>(reinterpret_cast<bf16*>(p.y) + pix * p.y_cstride + n);
+          yp[0] = make_uint4(w[0], w[1], w[2], w[3]);
+          yp[1] = make_uint4(w[4], w[5], w[6], w[7]);
+        }
+      } else {
+        // ragged / unaligned channel tail (e.g. Cout = 3): scalar path
+#pragma unroll
+        for (int j = 0; j < 16; ++j) {
+          const int nn = n + j;
+          if (nn < p.Cout) {
+            float x = f[j];
+            if (p.bias) x += __ldg(p.bias + nn);
+            if (res_pre) x = fmaf(__bfloat162float(p.residual[rpix * p.res_cstride + nn]), rs, x);
+            if (p.relu) x = fmaxf(x, 0.f);
+            if (p.mask) x = __bfloat162float(p.mask[pix * p.mask_cstride + nn]) > 0.f ? x : 0.f;
+            if (res_post) x = fmaf(__bfloat162float(p.residual[rpix * p.res_cstride + nn]), rs, x);
+            if (p.y_fp32) reinterpret_cast<float*>(p.y)[pix * p.y_cstride + nn] = x;
+            else reinterpret_cast<bf16*>(p.y)[pix * p.y_cstride + nn] = __float2bfloat16_rn(x);
           }
         }
       }
-      if (do_relu) {
-#pragma unroll
-        for (int j = 0; j < 16; ++j) f[j] = fmaxf(f[j], 0.f);
-        if constexpr ((F & kEpiBitsOut) != 0)
-          reinterpret_cast<unsigned short*>(p.relu_bits)[(pix * (p.Cout >> 6) + (n >> 6)) * 4 + ((n >> 4) & 3)] =
-              (unsigned short)positive_bits16(f);
-      }
-      if constexpr (has_mask && (F & kEpiMaskBits) != 0) {
-        apply_bits16(f, __ldg(reinterpret_cast<const unsigned short*>(p.mask_bits) + (pix * (p.Cout >> 6) + (n >> 6)) * 4 + ((n >> 4) & 3)));
-      } else if constexpr (has_mask) {
-        const uint4* mp = reinterpret_cast<const uint4*>(p.mask + pix * p.mask_cstride + n);
-#pragma unroll
-        for (int j = 0; j < 2; ++j) {
-          const uint4 m = __ldg(mp + j);
-          f[8 * j + 0] = bf16_bits_lo(m.x) > 0.f ? f[8 * j + 0] : 0.f;
-          f[8 * j + 1] = bf16_bits_hi(m.x) > 0.f ? f[8 * j + 1] : 0.f;
-          f[8 * j + 2] = bf16_bits_lo(m.y) > 0.f ? f[8 * j + 2] : 0.f;
-          f[8 * j + 3] = bf16_bits_hi(m.y) > 0.f ? f[8 * j + 3] : 0.f;
-          f[8 * j + 4] = bf16_bits_lo(m.z) > 0.f ? f[8 * j + 4] : 0.f;
-          f[8 * j + 5] = bf16_bits_hi(m.z) > 0.f ? f[8 * j + 5] : 0.f;
-          f[8 * j + 6] = bf16_bits_lo(m.w) > 0.f ? f[8 * j + 6] : 0.f;
-          f[8 * j + 7] = bf16_bits_hi(m.w) > 0.f ? f[8 * j + 7] : 0.f;
-        }
-      }
-      if (res_post) {
-        const uint4* rp = reinterpret_cast<const uint4*>(p.residual + rpix * p.res_cstride + n);
-#pragma unroll
-        for (int j = 0; j < 2; ++j) {
-          const uint4 r = __ldg(rp + j);
-          f[8 * j + 0] = fmaf(bf16_bits_lo(r.x), rs, f[8 * j + 0]); f[8 * j + 1] = fmaf(bf16_bits_hi(r.x), rs, f[8 * j + 1]);
-          f[8 * j + 2] = fmaf(bf16_bits_lo(r.y), rs, f[8 * j + 2]); f[8 * j + 3] = fmaf(bf16_bits_hi(r.y), rs, f[8 * j + 3]);
-          f[8 * j + 4] = fmaf(bf16_bits_lo(r.z), rs, f[8 * j + 4]); f[8 * j + 5] = fmaf(bf16_bits_hi(r.z), rs, f[8 * j + 5]);
-          f[8 * j + 6] = fmaf(bf16_bits_lo(r.w), rs, f[8 * j + 6]); f[8 * j + 7] = fmaf(bf16_bits_hi(r.w), rs, f[8 * j + 7]);
-        }
-      }
-      uint4* yp = reinterpret_cast<uint4*>(yrow + n);
-      yp[0] = make_uint4(pack_bf16x2(f[0], f[1]), pack_bf16x2(f[2], f[3]), pack_bf16x2(f[4], f[5]), pack_bf16x2(f[6], f[7]));
-      yp[1] = make_uint4(pack_bf16x2(f[8], f[9]), pack_bf16x2(f[10], f[11]), pack_bf16x2(f[12], f[13]), pack_bf16x2(f[14], f[15]));
     }
   }
 }
 
-// t_row : TMEM address (lane quadrant of this warp, first column of the accumulator).
+// Staged-store epilogue.  t_row: TMEM address (lane quadrant of this warp, first column of the accumulator).
 // c1..c3: box coordinates (w0, h0, b0) of the tile in the output tensor map; channel coordinate = n0 + chunk * 64.
-// stage : this team's staging buffer (1024-byte aligned).  team in {0,1}; row = accumulator row of this thread.
-// NH: warps per (team, lane quadrant).  1: a thread converts all four 16-column pieces of its row of the chunk; 2: two warps share
-// the row (``half`` 0 / 1 takes pieces 0-1 / 2-3), a team is 8 warps -- twice the warps per scheduler to hide the TMEM-load /
-// shared-memory latencies of the per-piece chain (r02 ncu of a 1x1 launch: 3 warps per scheduler, one eligible 46 % of cycles).
-template <int F, int NH = 1>
+// stage : this team's first staging tile (1024-byte aligned).  team in {0,1}; row = accumulator row of this thread.
+// sbuf != nullptr: the team owns two staging tiles used in turn, so a chunk only waits for the store issued two chunks ago --
+// the latency of the previous tensor store is off the critical path and more bytes are in flight; nullptr: one tile.
+template <int F>
 __device__ __forceinline__ void epilogue_tile_tma(const EpiArgs& p, const CUtensorMap* tmY, uint32_t t_row, int BN, int n0,
                                                   int c1, int c2, int c3, bool valid, long long pix, long long rpix, float alpha,
                                                   uint32_t stage, int team, int row, bool leader, int chunk_stride = 2,
-                                                  const EpiAux* aux = nullptr, uint32_t* sbuf = nullptr, int nbuf = 2, int half = 0) {
-  constexpr int kTeamThreads = 128 * NH;
-  const int sbeg = half * (4 / NH), send = sbeg + 4 / NH;
+                                                  const EpiAux* aux = nullptr, uint32_t* sbuf = nullptr) {
+  constexpr int kTeamThreads = 128;
   constexpr bool sm_apply = F >= 0 && (F & kEpiSmApply) != 0, sm_bwd = F >= 0 && (F & kEpiSmBwd) != 0;
   constexpr float kLog2e = 1.4426950408889634f;
   float sm_a = 0.f, sm_b = 1.f;                    // apply: (row max, 1 / row sum); backward: (delta, -)
@@ -406,8 +340,6 @@ __device__ __forceinline__ void epilogue_tile_tma(const EpiArgs& p, const CUtens
   const long long nw = p.Cout >> 6;
   const bool full_c = F >= 0 && (F & kEpiFull) != 0;       // no channel-tail tests
   const float rs = p.res_scale;
-  // sbuf != nullptr: the team owns ``nbuf`` (2..4) staging tiles used round-robin, so a chunk only waits for the store issued
-  // nbuf chunks ago -- the latency of the previous tensor stores is off the critical path and more bytes are in flight.
   const uint32_t sw = (uint32_t)(row & 7);
   // 1: residual tile via TMA, 2: mask tile via TMA (compile-time for F >= 0: the host sets the aux bits iff it passes ``aux``)
   const int aux_kind = F < 0 ? ((aux && (res_pre || res_post || has_mask)) ? aux->kind : 0)
@@ -418,22 +350,16 @@ __device__ __forceinline__ void epilogue_tile_tma(const EpiArgs& p, const CUtens
     if (nbase >= p.Cout) break;
     uint32_t mlo = 0u, mhi = 0u, olo = 0u, ohi = 0u;
     if (use_mbits && valid) {                    // 8 bytes instead of a 128-byte line of the bf16 activation
-      if (NH == 1) {
-        const uint2 m = __ldg(reinterpret_cast<const uint2*>(p.mask_bits) + pix * nw + (nbase >> 6));
-        mlo = m.x; mhi = m.y;
-      } else {
-        mlo = mhi = __ldg(reinterpret_cast<const uint32_t*>(p.mask_bits) + (pix * nw + (nbase >> 6)) * 2 + half);
-      }
+      const uint2 m = __ldg(reinterpret_cast<const uint2*>(p.mask_bits) + pix * nw + (nbase >> 6));
+      mlo = m.x; mhi = m.y;
     }
     const uint32_t stage_cur = stage + (sbuf ? *sbuf * kEpiStageBytes : 0u);
     const uint32_t srow = stage_cur + (uint32_t)row * 128u;
     if (leader) {                                // the store that last used this staging tile has finished reading it
       if (!sbuf) bulk_wait_read0();
-      else if (nbuf == 2) bulk_wait_read1();
-      else if (nbuf == 3) bulk_wait_read2();
-      else bulk_wait_read3();
+      else bulk_wait_read1();
     }
-    if (sbuf) *sbuf = (*sbuf + 1u == (uint32_t)nbuf) ? 0u : *sbuf + 1u;
+    if (sbuf) *sbuf ^= 1u;
     named_bar_sync(1 + team, kTeamThreads);
     uint32_t arow_addr = 0u, aslot = 0u;
     if (aux_kind) {                              // residual / mask chunk: one TMA box (fetched ahead by the aux producer warp)
@@ -453,6 +379,13 @@ __device__ __forceinline__ void epilogue_tile_tma(const EpiArgs& p, const CUtens
         for (int j = 0; j < 16; ++j) f[j] = __uint_as_float(v[j]) * alpha;
         const int nvalid = full_c ? 16 : p.Cout - n;   // channels of this 16-wide piece inside the tensor: >= 16, 8 (Cout % 16 == 8) or <= 0
         const bool in_c = full_c || nvalid > 0;
+        // 16-byte unit j (0, 1) of this piece in a bf16 operand: this row of the aux tile when the operand rides the ring
+        // (unit u of a 128-byte line lives at u ^ (row & 7)), else a direct load, zeros past the channel tail
+        auto unit = [&](const bf16* base, int kind, int j) -> uint4 {
+          return (aux_kind == kind) ? ld_shared_v4(arow_addr + (((uint32_t)(2 * s + j) ^ asw) << 4))
+                                    : ((full_c || 8 * j < nvalid) ? __ldg(reinterpret_cast<const uint4*>(base) + j)
+                                                                  : make_uint4(0u, 0u, 0u, 0u));
+        };
         if (sm_apply) {
 #pragma unroll
           for (int j = 0; j < 16; ++j) f[j] = fast_ex2(fmaf(f[j], kLog2e, sm_a)) * sm_b;
@@ -467,27 +400,10 @@ __device__ __forceinline__ void epilogue_tile_tma(const EpiArgs& p, const CUtens
             f[8 * j + 6] = bf16_bits_lo(r.w) * (f[8 * j + 6] - sm_a); f[8 * j + 7] = bf16_bits_hi(r.w) * (f[8 * j + 7] - sm_a);
           }
         }
-        if (has_bias && in_c) {
-          const float4* bp = reinterpret_cast<const float4*>(p.bias + n);
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            if (full_c || 4 * j < nvalid) {
-              const float4 bb = __ldg(bp + j);
-              f[4 * j + 0] += bb.x; f[4 * j + 1] += bb.y; f[4 * j + 2] += bb.z; f[4 * j + 3] += bb.w;
-            }
-          }
-        }
+        if (has_bias && in_c) piece_bias(f, p.bias + n, nvalid);
         if (res_pre && in_c && valid) {
-          const uint4* rp = reinterpret_cast<const uint4*>(p.residual + rpix * p.res_cstride + n);
-#pragma unroll
-          for (int j = 0; j < 2; ++j) {
-            const uint4 r = (aux_kind == 1) ? ld_shared_v4(arow_addr + (((uint32_t)(2 * s + j) ^ asw) << 4))
-                                            : ((full_c || 8 * j < nvalid) ? __ldg(rp + j) : make_uint4(0u, 0u, 0u, 0u));
-            f[8 * j + 0] = fmaf(bf16_bits_lo(r.x), rs, f[8 * j + 0]); f[8 * j + 1] = fmaf(bf16_bits_hi(r.x), rs, f[8 * j + 1]);
-            f[8 * j + 2] = fmaf(bf16_bits_lo(r.y), rs, f[8 * j + 2]); f[8 * j + 3] = fmaf(bf16_bits_hi(r.y), rs, f[8 * j + 3]);
-            f[8 * j + 4] = fmaf(bf16_bits_lo(r.z), rs, f[8 * j + 4]); f[8 * j + 5] = fmaf(bf16_bits_hi(r.z), rs, f[8 * j + 5]);
-            f[8 * j + 6] = fmaf(bf16_bits_lo(r.w), rs, f[8 * j + 6]); f[8 * j + 7] = fmaf(bf16_bits_hi(r.w), rs, f[8 * j + 7]);
-          }
+          const bf16* rrow = p.residual + rpix * p.res_cstride + n;
+          piece_res_fma(f, unit(rrow, 1, 0), unit(rrow, 1, 1), rs);
         }
         uint32_t ob = 0u;
         if (do_relu) {
@@ -498,44 +414,23 @@ __device__ __forceinline__ void epilogue_tile_tma(const EpiArgs& p, const CUtens
         if (use_mbits) {
           apply_bits16(f, mb);
         } else if (has_mask && in_c && valid) {
-          const uint4* mp = reinterpret_cast<const uint4*>(p.mask + pix * p.mask_cstride + n);
-#pragma unroll
-          for (int j = 0; j < 2; ++j) {
-            const uint4 m = (aux_kind == 2) ? ld_shared_v4(arow_addr + (((uint32_t)(2 * s + j) ^ asw) << 4))
-                                            : ((full_c || 8 * j < nvalid) ? __ldg(mp + j) : make_uint4(0u, 0u, 0u, 0u));
-            f[8 * j + 0] = bf16_bits_lo(m.x) > 0.f ? f[8 * j + 0] : 0.f;
-            f[8 * j + 1] = bf16_bits_hi(m.x) > 0.f ? f[8 * j + 1] : 0.f;
-            f[8 * j + 2] = bf16_bits_lo(m.y) > 0.f ? f[8 * j + 2] : 0.f;
-            f[8 * j + 3] = bf16_bits_hi(m.y) > 0.f ? f[8 * j + 3] : 0.f;
-            f[8 * j + 4] = bf16_bits_lo(m.z) > 0.f ? f[8 * j + 4] : 0.f;
-            f[8 * j + 5] = bf16_bits_hi(m.z) > 0.f ? f[8 * j + 5] : 0.f;
-            f[8 * j + 6] = bf16_bits_lo(m.w) > 0.f ? f[8 * j + 6] : 0.f;
-            f[8 * j + 7] = bf16_bits_hi(m.w) > 0.f ? f[8 * j + 7] : 0.f;
-          }
+          const bf16* mrow = p.mask + pix * p.mask_cstride + n;
+          piece_mask_bf16(f, unit(mrow, 2, 0), unit(mrow, 2, 1));
         }
         if (res_post && in_c && valid) {
-          const uint4* rp = reinterpret_cast<const uint4*>(p.residual + rpix * p.res_cstride + n);
-#pragma unroll
-          for (int j = 0; j < 2; ++j) {
-            const uint4 r = (aux_kind == 1) ? ld_shared_v4(arow_addr + (((uint32_t)(2 * s + j) ^ asw) << 4))
-                                            : ((full_c || 8 * j < nvalid) ? __ldg(rp + j) : make_uint4(0u, 0u, 0u, 0u));
-            f[8 * j + 0] = fmaf(bf16_bits_lo(r.x), rs, f[8 * j + 0]); f[8 * j + 1] = fmaf(bf16_bits_hi(r.x), rs, f[8 * j + 1]);
-            f[8 * j + 2] = fmaf(bf16_bits_lo(r.y), rs, f[8 * j + 2]); f[8 * j + 3] = fmaf(bf16_bits_hi(r.y), rs, f[8 * j + 3]);
-            f[8 * j + 4] = fmaf(bf16_bits_lo(r.z), rs, f[8 * j + 4]); f[8 * j + 5] = fmaf(bf16_bits_hi(r.z), rs, f[8 * j + 5]);
-            f[8 * j + 6] = fmaf(bf16_bits_lo(r.w), rs, f[8 * j + 6]); f[8 * j + 7] = fmaf(bf16_bits_hi(r.w), rs, f[8 * j + 7]);
-          }
+          const bf16* rrow = p.residual + rpix * p.res_cstride + n;
+          piece_res_fma(f, unit(rrow, 1, 0), unit(rrow, 1, 1), rs);
         }
         // 16 channels = two 16-byte units (2s, 2s+1) of this row's 128-byte line; unit u lives at (u ^ (row & 7))
         uint32_t w[8];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) w[j] = pack_bf16x2(f[2 * j], f[2 * j + 1]);
+        piece_pack(f, w);
         if (bits_from_packed) ob = positive_bits16_packed(w);
         st_shared_v4(srow + (((uint32_t)(2 * s) ^ sw) << 4), w[0], w[1], w[2], w[3]);
         st_shared_v4(srow + (((uint32_t)(2 * s + 1) ^ sw) << 4), w[4], w[5], w[6], w[7]);
         return ob;
     };
 #pragma unroll 1
-    for (int s0 = sbeg; s0 < send; s0 += NP) {
+    for (int s0 = 0; s0 < 4; s0 += NP) {
       uint32_t v[NP][16];
       __syncwarp();
 #pragma unroll
@@ -549,10 +444,7 @@ __device__ __forceinline__ void epilogue_tile_tma(const EpiArgs& p, const CUtens
         else ohi |= ob << (16 * (s & 1));
       }
     }
-    if (emit_bits && valid) {
-      if (NH == 1) reinterpret_cast<uint2*>(p.relu_bits)[pix * nw + (nbase >> 6)] = make_uint2(olo, ohi);
-      else reinterpret_cast<uint32_t*>(p.relu_bits)[(pix * nw + (nbase >> 6)) * 2 + half] = half ? ohi : olo;
-    }
+    if (emit_bits && valid) reinterpret_cast<uint2*>(p.relu_bits)[pix * nw + (nbase >> 6)] = make_uint2(olo, ohi);
     fence_proxy_async_smem();                    // generic-proxy smem writes -> visible to the TMA (async proxy)
     named_bar_sync(1 + team, kTeamThreads);
     if (leader) {

@@ -84,8 +84,6 @@ __device__ __forceinline__ void tma_store_4d(const CUtensorMap* m, uint32_t src,
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait_read1() { asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_read2() { asm volatile("cp.async.bulk.wait_group.read 2;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_read3() { asm volatile("cp.async.bulk.wait_group.read 3;" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 __device__ __forceinline__ void named_bar_sync(uint32_t id, uint32_t nthreads) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");

@@ -10,8 +10,6 @@
 // One persistent CTA per SM, 6 warps: warp 0 = TMA producer (one lane), warp 1 = tcgen05.mma issuer (one lane) and
 // TMEM owner, warps 2..5 = epilogue (TMEM -> registers -> fused epilogue -> global).  Two TMEM accumulator stages so
 // the epilogue of tile i overlaps the main loop of tile i+1.
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "ptx.cuh"
 #include "conv_epilogue.cuh"
@@ -19,12 +17,7 @@
 namespace sgb {
 
 static constexpr int kWgradThreads = 192;                // wgrad: warps 0 producer, 1 MMA, 2..5 epilogue
-#ifndef SGB_FPROP_NH
-#define SGB_FPROP_NH 1                               // warps per (team, lane quadrant) in the epilogue; 2 = 16 epilogue warps (A/B on one box, r02: 565.1 vs 563.2 ms/step -- no gain, the 1x1 launches sit on the HBM read/write mix, not on epilogue latency)
-#endif
-static constexpr int kFpropNH = SGB_FPROP_NH;
-static constexpr int kFpropEpiThreads = 256 * kFpropNH;   // 2 teams x 4 lane quadrants x NH column halves
-static constexpr int kThreads = 128 + kFpropEpiThreads;  // warps 0..3: producer / MMA / aux producer / (idle), warps 4..19: epilogue teams
+static constexpr int kThreads = 128 + kEpiThreads;       // warps 0..3: producer / MMA / aux producer / (idle), warps 4..11: epilogue teams
 static constexpr int kTileM = 128;          // pixels (fprop) or output channels (wgrad) per tile = TMEM lanes
 static constexpr int kBlockK = 64;          // bf16 elements per 128-byte swizzle row
 static constexpr int kABytes = kTileM * kBlockK * 2;  // 16 KiB
@@ -38,7 +31,7 @@ struct FpropArgs {
   int w_mode;                     // 0: shared weights [Cout][taps][Cin]; 1: per-image [B][N][K]; 2: per-image MN-major [B][K][N]
   int stages;
   int use_tma;                    // epilogue through staging tiles + TMA tensor stores
-  int epi_nbuf;                   // staging tiles per epilogue team (2..4: stores overlap the next chunks' conversion)
+  int epi_nbuf;                   // staging tiles per epilogue team (2: a store overlaps the next chunk's conversion)
   int b_resident;                 // 1: every weight tile of this CTA's channel tile stays in shared memory (loaded once)
   int aux_kind, aux_tw, aux_th;   // residual (1) / mask (2) tile staged by TMA; its box is aux_tw x aux_th x nb pixels
   int aux_depth;                  // aux tiles per epilogue team (ring filled by the aux producer warp)
@@ -80,7 +73,7 @@ conv_fprop_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
     }
     for (int a = 0; a < 2; ++a) {
       mbar_init(tfull_bar(a), 1);
-      mbar_init(tempty_bar(a), kFpropEpiThreads);
+      mbar_init(tempty_bar(a), kEpiThreads);
       for (int sl = 0; sl < p.aux_depth; ++sl) { mbar_init(aux_full(a, sl), 1); mbar_init(aux_empty(a, sl), 1); }
     }
     mbar_init(bres_bar, 1);
@@ -198,13 +191,12 @@ conv_fprop_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
       }
     }
   } else if (warp >= 4) {
-    // --------------------------------------------------------------- epilogue: 16 warps, TMEM lane quadrant = warp % 4;
-    // team = which 64-channel chunks (even / odd), half = which two of the four 16-column pieces of a chunk
+    // --------------------------------------------------------------- epilogue: 8 warps, TMEM lane quadrant = warp % 4;
+    // team = which 64-channel chunks (even / odd)
     const int q = warp & 3;
-    const int team = ((warp - 4) >> 2) & 1;
-    const int half = (warp - 4) >> 3;
+    const int team = (warp - 4) >> 2;
     const int row = q * 32 + lane;
-    const bool leader = (q == 0) && (lane == 0) && (half == 0);
+    const bool leader = (q == 0) && (lane == 0);
     const int wi = row % p.tw, hi = (row / p.tw) % p.th, bi = row / (p.tw * p.th);
     const bool vec_ok = epi_vec_ok(p.e);
     const float alpha = p.e.alpha_ptr ? p.e.alpha * __ldg(p.e.alpha_ptr) : p.e.alpha;
@@ -234,12 +226,12 @@ conv_fprop_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
       tc_fence_after();
       const uint32_t t_row = tmem_base + ((uint32_t)(q * 32) << 16) + a * p.BN;
       if constexpr (F >= 0 && (F & kEpiSmStats) != 0) {
-        if (half == 0) epilogue_tile_smstats(p.e, t_row, p.BN, n0, valid, pix, alpha, team, nt * 2 + team);
-      } else if (p.use_tma) {
-        epilogue_tile_tma<F, kFpropNH>(p.e, &tmY, t_row, p.BN, n0, wt * p.tw, ht * p.th, bt * p.nb, valid, pix, rpix, alpha, stage, team, row,
-                             leader, 2, p.aux_kind ? &aux : nullptr, p.epi_nbuf >= 2 ? &sbuf : nullptr, p.epi_nbuf, half);
-      } else if (team == 0 && half == 0) {
-        epilogue_row(p.e, t_row, p.BN, n0, valid, pix, rpix, alpha, vec_ok);
+        epilogue_tile_smstats(p.e, t_row, p.BN, n0, valid, pix, alpha, team, nt * 2 + team);
+      } else if (F >= 0 || p.use_tma) {          // (the host picks a compile-time variant only for staged stores)
+        epilogue_tile_tma<F>(p.e, &tmY, t_row, p.BN, n0, wt * p.tw, ht * p.th, bt * p.nb, valid, pix, rpix, alpha, stage, team, row,
+                             leader, 2, p.aux_kind ? &aux : nullptr, p.epi_nbuf == 2 ? &sbuf : nullptr);
+      } else if (team == 0) {
+        epilogue_row<F>(p.e, t_row, p.BN, n0, valid, pix, rpix, alpha, vec_ok);
       }
       tc_fence_before();
       mbar_arrive(tempty_bar(a));
@@ -489,23 +481,13 @@ namespace sgb {
 bool wgrad3x3_c64_eligible(const sgb_wgrad_desc* d);
 int launch_wgrad3x3_c64(const sgb_wgrad_desc* d, cudaStream_t stream);
 bool conv3x3_rows_eligible(const sgb_conv_desc* d);
-int launch_conv3x3_rows(const sgb_conv_desc* d, cudaStream_t stream, int bo_mode, int use_tma_env);
+int launch_conv3x3_rows(const sgb_conv_desc* d, cudaStream_t stream);
 }  // namespace sgb
 
-static int env_int(const char* name, int dflt) {
-  const char* v = getenv(name);
-  return v ? atoi(v) : dflt;
-}
-// Bring-up switches: read from the environment ONCE per process (a conv launch used to call getenv five times).
-struct EngineSwitches {
-  int conv3x3_rows, rows_base_offset, epi_tma, epi_tma_maxk, epi_aux, epi_nbuf, wgrad3x3, b_resident, aux_depth;
-};
-static const EngineSwitches& switches() {
-  static const EngineSwitches s = {env_int("SGB_CONV3X3_ROWS", 1), env_int("SGB_ROWS_BASE_OFFSET", 0), env_int("SGB_EPI_TMA", 1),
-                                   env_int("SGB_EPI_TMA_MAXK", 640), env_int("SGB_EPI_AUX", 1), env_int("SGB_EPI_NBUF", 2),
-                                   env_int("SGB_WGRAD3X3", 1), env_int("SGB_B_RESIDENT", 1), env_int("SGB_AUX_DEPTH", 2)};
-  return s;
-}
+// The staged-store epilogue serves the output-heavy layers: K = taps * Cin up to this.  Longer-K layers store directly and
+// keep the shared memory of the staging tiles for operand stages.
+static constexpr int kEpiTmaMaxK = 640;
+static constexpr int kAuxDepth = 2;       // aux ring tiles per epilogue team (profiles/r02_aux_depth_sweep.txt: 3 is no faster)
 
 template <int F>
 static int launch_fprop(int grid, size_t smem, cudaStream_t stream, const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmY,
@@ -566,17 +548,12 @@ extern "C" int sgb_conv_fprop(const sgb_conv_desc* d, sgb_stream_t stream_) {
   // attention softmax inside the epilogue: plain bf16 GEMM tiles only
   SGB_REQUIRE(d->sm_mode >= 0 && d->sm_mode <= 3);
   SGB_REQUIRE(!d->sm_mode || (d->Cout % 64 == 0 && !d->y_fp32 && d->out_sub != 2 && !d->bias && !d->residual && !d->mask && !d->mask_bits &&
-                              !d->relu && d->KH == 1 && d->KW == 1 && d->Cin <= 640 && d->y_cstride % 8 == 0));
+                              !d->relu && d->KH == 1 && d->KW == 1 && d->Cin <= kEpiTmaMaxK && d->y_cstride % 8 == 0));
   SGB_REQUIRE(d->sm_mode != 1 || d->sm_stats);
   SGB_REQUIRE(d->sm_mode != 2 || d->sm_stats);
   SGB_REQUIRE(d->sm_mode != 3 || (d->sm_delta && d->sm_p && d->sm_p_cstride % 8 == 0 && ((uintptr_t)d->sm_p & 15) == 0));
-  {
-    // wide, few-channel 3x3 layers: halo-row kernel (umma_conv3x3.cu).  SGB_CONV3X3_ROWS=0 forces the generic kernel.
-    const EngineSwitches& sw = switches();
-    if (sw.conv3x3_rows && d->Hin <= 0 && d->Win <= 0 && d->out_sub != 2 && conv3x3_rows_eligible(d))
-      return launch_conv3x3_rows(d, stream, sw.rows_base_offset, sw.epi_tma);
-  }
-  SGB_REQUIRE(((uintptr_t)d->bias & 15) == 0 && ((uintptr_t)d->residual & 15) == 0 && ((uintptr_t)d->mask & 15) == 0);
+  // wide, few-channel 3x3 layers: halo-row kernel (umma_conv3x3.cu)
+  if (d->Hin <= 0 && d->Win <= 0 && d->out_sub != 2 && conv3x3_rows_eligible(d)) return launch_conv3x3_rows(d, stream);
 
   FpropArgs p;
   p.B = d->B; p.H = d->H; p.W = d->W; p.Cin = d->Cin; p.Cout = d->Cout;
@@ -594,12 +571,12 @@ extern "C" int sgb_conv_fprop(const sgb_conv_desc* d, sgb_stream_t stream_) {
   const int Hin = d->Hin > 0 ? d->Hin : d->H, Win = d->Win > 0 ? d->Win : d->W;
   p.out_sub = d->out_sub == 2 ? 2 : 1;
   SGB_REQUIRE(p.out_sub == 1 || (!d->residual && !d->mask));
-  p.use_tma = (p.out_sub == 1 && !d->y_fp32 && BN % 64 == 0 && d->Cout % 8 == 0 && d->y_cstride % 8 == 0 &&
-               (!d->residual || d->res_cstride % 8 == 0) && (!d->mask || d->mask_cstride % 8 == 0) &&
-               p.taps * d->Cin <= switches().epi_tma_maxk && switches().epi_tma) ? 1 : 0;   // output-heavy layers only
+  fill_epi(p.e, d);
+  p.e.sm_parts = 2 * p.tiles_n;
+  p.use_tma = (p.out_sub == 1 && epi_can_stage(p.e, BN) && p.taps * d->Cin <= kEpiTmaMaxK) ? 1 : 0;
   // auxiliary epilogue operand through TMA: exactly one of residual / mask, bf16 NHWC with 16-byte aligned channel stride
   p.aux_kind = 0; p.aux_tw = p.tw; p.aux_th = p.th;
-  if (p.use_tma && switches().epi_aux && (d->residual != nullptr || d->mask != nullptr)) {   // (mask_bits are 8-byte direct loads)
+  if (p.use_tma && (d->residual != nullptr || d->mask != nullptr)) {   // (mask_bits are 8-byte direct loads)
     // one operand rides TMA: the mask when both are present (full-resolution tile; the residual of such launches is the
     // quarter-size pooled-skip gradient, whose direct 16-byte loads are shared by 2x2 pixel neighbours through L1)
     if (d->mask) p.aux_kind = 2;
@@ -615,11 +592,10 @@ extern "C" int sgb_conv_fprop(const sgb_conv_desc* d, sgb_stream_t stream_) {
   // space of the B halves of the ring buys more staging tiles per epilogue team = more store bytes in flight
   const uint32_t b_tile = (uint32_t)BN * kBlockK * 2;
   const int kt = p.taps * p.kblocks;
-  p.b_resident = (switches().b_resident && d->w_mode == 0 && p.tiles_n == 1 && kt <= 2 && kt * b_tile <= 64u * 1024u) ? 1 : 0;
+  p.b_resident = (d->w_mode == 0 && p.tiles_n == 1 && kt <= 2 && kt * b_tile <= 64u * 1024u) ? 1 : 0;
   const uint32_t stage_bytes = kABytes + (p.b_resident ? 0u : b_tile);
-  const int nbuf_want = switches().epi_nbuf < 1 ? 1 : (switches().epi_nbuf > 4 ? 4 : switches().epi_nbuf);
-  p.epi_nbuf = (p.use_tma && kt <= 2) ? nbuf_want : 1;
-  p.aux_depth = p.aux_kind ? (switches().aux_depth < 1 ? 1 : (switches().aux_depth > 3 ? 3 : switches().aux_depth)) : 1;
+  p.epi_nbuf = (p.use_tma && kt <= 2) ? 2 : 1;
+  p.aux_depth = p.aux_kind ? kAuxDepth : 1;
   auto ring_kb = [&](int nbuf) { return 216 - (p.use_tma ? 32 * nbuf : 0) - (p.aux_kind ? 32 * p.aux_depth : 0) - (p.b_resident ? (int)(kt * b_tile / 1024) : 0); };
   // keep >= 3 operand ring stages: give back aux depth first, then staging tiles
   while (p.aux_kind && p.aux_depth > 1 && ring_kb(p.epi_nbuf) * 1024 < (int)(3 * stage_bytes)) --p.aux_depth;
@@ -629,8 +605,6 @@ extern "C" int sgb_conv_fprop(const sgb_conv_desc* d, sgb_stream_t stream_) {
   if (stages < 2) stages = 2;
   p.stages = stages;
   p.tmem_cols = pow2_cols(2 * BN);
-  fill_epi(p.e, d);
-  p.e.sm_parts = 2 * p.tiles_n;
 
   CUtensorMap tmA, tmB;
   int rc = make_act_tmap(&tmA, d->x, d->B, Hin, Win, d->Cin, d->x_cstride, p.tw, p.th, p.nb);
@@ -666,7 +640,7 @@ extern "C" int sgb_conv_fprop(const sgb_conv_desc* d, sgb_stream_t stream_) {
     if (rc) return rc;
   }
   const size_t smem = (size_t)stages * stage_bytes + (p.use_tma ? 2 * p.epi_nbuf * kEpiStageBytes : 0) + (p.aux_kind ? 2 * p.aux_depth * kEpiStageBytes : 0) +
-                      (p.b_resident ? (size_t)kt * b_tile : 0) + 1024 + 8 * (2 * stages + 8 + 4 * 3) + 16;
+                      (p.b_resident ? (size_t)kt * b_tile : 0) + 1024 + 8 * (2 * stages + 8 + 4 * kAuxDepth) + 16;
   int grid = p.num_tiles < sm_count() ? p.num_tiles : sm_count();
   // the hot epilogue shapes of the training step get compile-time variants; everything else takes the general kernel
   int f = p.use_tma ? epi_flags_of(p.e) : -1;
@@ -698,7 +672,7 @@ extern "C" int sgb_conv_fprop(const sgb_conv_desc* d, sgb_stream_t stream_) {
 
 extern "C" int sgb_conv_wgrad_fuses_dbias(const sgb_wgrad_desc* d) {
   if (!d) return 0;
-  if (switches().wgrad3x3 && wgrad3x3_c64_eligible(d)) return 1;
+  if (wgrad3x3_c64_eligible(d)) return 1;
   return d->per_image ? 0 : 1;          // generic kernel: constant-ones B operand on its (first channel tile, first tap) items
 }
 
@@ -708,7 +682,7 @@ extern "C" int sgb_conv_wgrad(const sgb_wgrad_desc* d, sgb_stream_t stream_) {
   SGB_REQUIRE(d->B > 0 && d->H > 0 && d->W > 0 && d->Cin > 0 && d->Cout > 0 && d->KH > 0 && d->KW > 0);
   SGB_REQUIRE(d->Cin % 8 == 0 && d->x_cstride % 8 == 0 && d->Cout % 8 == 0 && d->dy_cstride % 8 == 0);
   SGB_REQUIRE(((uintptr_t)d->x & 15) == 0 && ((uintptr_t)d->dy & 15) == 0);
-  if (switches().wgrad3x3 && wgrad3x3_c64_eligible(d)) return launch_wgrad3x3_c64(d, stream);
+  if (wgrad3x3_c64_eligible(d)) return launch_wgrad3x3_c64(d, stream);
   SGB_REQUIRE(d->dbias == nullptr || !d->per_image);
 
   WgradArgs p;

@@ -24,17 +24,11 @@ static constexpr int kRowsThreads = 128 + kEpiThreads;  // warps 0: A producer, 
 struct RowsArgs {
   int B, H, W, Cin, Cout;
   int kblocks, BN, tiles_n, segs, hpairs, num_tiles;
-  int resident, a_stages, b_stages, bo_mode;
+  int resident, a_stages, b_stages;
   int use_tma, epi_bufs;   // TMA-store epilogue; 2 staging tiles: team t owns output row t, 1: team 0 handles both rows
   uint32_t tmem_cols;
   EpiArgs e;
 };
-
-__device__ __forceinline__ uint64_t sdesc_rows(uint32_t addr, int bo_mode) {
-  uint64_t d = make_sdesc_sw128(addr, 16, 1024);
-  if (bo_mode) d |= (uint64_t)((addr >> 7) & 7u) << 49;   // matrix base offset (start not on a 1024-byte boundary)
-  return d;
-}
 
 template <int F>      // epilogue variant, see conv_epilogue.cuh
 __global__ void __launch_bounds__(kRowsThreads, 1)
@@ -152,7 +146,7 @@ conv3x3_rows_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
             for (int r = 1; r <= 2; ++r)
               for (int kw = 0; kw < 3; ++kw) {
                 const uint64_t bdesc = make_sdesc_sw128(b_base + ((kb * 3 + kw) * 3 + (r - 1)) * b_tile_bytes, 16, 1024);
-                const uint64_t adesc = sdesc_rows(sa + r * kRowBufBytes + kw * 128, p.bo_mode);
+                const uint64_t adesc = make_sdesc_sw128(sa + r * kRowBufBytes + kw * 128, 16, 1024);
 #pragma unroll
                 for (int kk = 0; kk < 4; ++kk)
                   umma_f16_ss(d_pair, adesc + 2 * kk, bdesc + 2 * kk, idesc2, (kb > 0 || r > 1 || kw > 0 || kk > 0) ? 1u : 0u);
@@ -160,7 +154,7 @@ conv3x3_rows_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
             for (int e = 0; e < 2; ++e)          // r = 0: tap row 0 -> output row 0;  r = 3: tap row 2 -> output row 1
               for (int kw = 0; kw < 3; ++kw) {
                 const uint64_t bdesc = make_sdesc_sw128(b_base + ((kb * 3 + kw) * 3 + (e ? 2 : 0)) * b_tile_bytes, 16, 1024);
-                const uint64_t adesc = sdesc_rows(sa + (e ? 3 : 0) * kRowBufBytes + kw * 128, p.bo_mode);
+                const uint64_t adesc = make_sdesc_sw128(sa + (e ? 3 : 0) * kRowBufBytes + kw * 128, 16, 1024);
                 const uint32_t d_one = d_pair + (e ? 0 : p.BN);
 #pragma unroll
                 for (int kk = 0; kk < 4; ++kk) umma_f16_ss(d_one, adesc + 2 * kk, bdesc + 2 * kk, idesc, 1u);
@@ -176,7 +170,7 @@ conv3x3_rows_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
             const uint64_t bdesc = make_sdesc_sw128(b_base + sb * b_tile_bytes, 16, 1024);
 #pragma unroll
             for (int j = 0; j < 2; ++j) {
-              const uint64_t adesc = sdesc_rows(sa + (kh + j) * kRowBufBytes + kw * 128, p.bo_mode);
+              const uint64_t adesc = make_sdesc_sw128(sa + (kh + j) * kRowBufBytes + kw * 128, 16, 1024);
               const uint32_t d_tmem = tmem_base + (as * 2 + j) * p.BN;
 #pragma unroll
               for (int kk = 0; kk < 4; ++kk)
@@ -212,7 +206,7 @@ conv3x3_rows_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         const long long pix = ((long long)b * p.H + h) * p.W + w;
         const long long rpix = p.e.res_up2 ? (((long long)b * (p.H >> 1) + (h >> 1)) * (p.W >> 1) + (w >> 1)) : pix;
         const uint32_t t_row = tmem_base + ((uint32_t)(q * 32) << 16) + (as * 2 + (p.resident ? 1 - j : j)) * p.BN;
-        if (p.use_tma) {
+        if (F >= 0 || p.use_tma) {               // (the host picks a compile-time variant only for staged stores)
           // team t owns output row t.  epi_bufs == 2: both teams stage + TMA-store; epi_bufs == 1 (no room for a second
           // staging tile, C = 64): team 0 stages + TMA-stores row 0 while team 1 writes row 1 with direct 16-byte stores
           // (one full 128-byte line per thread at C = 64) -- two rows drain concurrently instead of back to back.
@@ -222,12 +216,11 @@ conv3x3_rows_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
               // one team covers every chunk of its row: run the chunk loop for both parities on the team's own barrier
               epilogue_tile_tma<F>(p.e, &tmY, t_row, p.BN, nt * p.BN, ws * 128, h, b, true, pix, rpix, alpha, stage, team, row, leader, 1);
             } else {
-              if constexpr (F >= 0) epilogue_row_fast<F>(p.e, t_row, p.BN, nt * p.BN, true, pix, rpix, alpha);
-              else epilogue_row(p.e, t_row, p.BN, nt * p.BN, true, pix, rpix, alpha, vec_ok);
+              epilogue_row<F>(p.e, t_row, p.BN, nt * p.BN, true, pix, rpix, alpha, vec_ok);
             }
           }
         } else if (team == 0) {
-          epilogue_row(p.e, t_row, p.BN, nt * p.BN, true, pix, rpix, alpha, vec_ok);
+          epilogue_row<F>(p.e, t_row, p.BN, nt * p.BN, true, pix, rpix, alpha, vec_ok);
         }
       }
       tc_fence_before();
@@ -264,8 +257,7 @@ bool conv3x3_rows_eligible(const sgb_conv_desc* d) {
          d->Cin % 64 == 0 && d->Cin <= 128 && d->Cout % 8 == 0;
 }
 
-// bo_mode: 0 = no matrix base offset in the row-shifted descriptors (default), 1 = (addr >> 7) & 7.
-int launch_conv3x3_rows(const sgb_conv_desc* d, cudaStream_t stream, int bo_mode, int use_tma_env) {
+int launch_conv3x3_rows(const sgb_conv_desc* d, cudaStream_t stream) {
   RowsArgs p;
   p.B = d->B; p.H = d->H; p.W = d->W; p.Cin = d->Cin; p.Cout = d->Cout;
   p.kblocks = d->Cin / 64;
@@ -274,13 +266,12 @@ int launch_conv3x3_rows(const sgb_conv_desc* d, cudaStream_t stream, int bo_mode
   p.segs = d->W / 128;
   p.hpairs = d->H / 2;
   p.num_tiles = p.tiles_n * p.segs * p.hpairs * d->B;
-  p.bo_mode = bo_mode;
+  fill_epi(p.e, d);
   const uint32_t b_tile = p.BN * 128u;
   const uint32_t budget = 227u * 1024u - 2048u;
   const uint32_t a_stage = 4 * kRowBufBytes;
   const uint32_t resident_bytes = 9u * p.kblocks * b_tile;
-  p.use_tma = (!d->y_fp32 && p.BN % 64 == 0 && d->y_cstride % 8 == 0 && (!d->residual || d->res_cstride % 8 == 0) &&
-               (!d->mask || d->mask_cstride % 8 == 0) && use_tma_env) ? 1 : 0;
+  p.use_tma = epi_can_stage(p.e, p.BN) ? 1 : 0;
   p.epi_bufs = 2;
   p.resident = (p.tiles_n == 1 && resident_bytes + 2 * a_stage + (p.use_tma ? kEpiStageBytes : 0) <= budget) ? 1 : 0;
   if (p.resident) {
@@ -299,7 +290,6 @@ int launch_conv3x3_rows(const sgb_conv_desc* d, cudaStream_t stream, int bo_mode
   uint32_t cols = 32;
   while ((int)cols < 4 * p.BN) cols <<= 1;
   p.tmem_cols = cols;
-  fill_epi(p.e, d);
 
   CUtensorMap tmA, tmB;
   {

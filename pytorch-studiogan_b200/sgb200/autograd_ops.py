@@ -7,7 +7,6 @@ Conventions
   (the consumer's dgrad epilogue does it for free via ``mask_input=True``).  That gradient is therefore the
   gradient w.r.t. the pre-activation and is used as is.
 """
-import os
 import torch
 import torch.distributed as dist
 from torch.autograd import Function
@@ -840,9 +839,6 @@ class ImageOutFn(TFunction):
         return K.img_grad_to_nhwc(dimg, img, ctx.Cp), None
 
 
-FUSED_SOFTMAX = os.environ.get("SGB_ATTN_FUSED_SOFTMAX", "1") != "0"   # A/B switch, read once
-
-
 class SelfAttentionFn(TFunction):
     """ops.SelfAttention.forward (src/utils/ops.py:83-103) with the attention map materialised in bf16:
        theta = conv(x), phi = maxpool(conv(x)), g = maxpool(conv(x)); P = softmax(theta . phi^T); o = P . g;
@@ -876,7 +872,7 @@ class SelfAttentionFn(TFunction):
         g_f = K.conv_fprop(x, packs[2][0], c2, 1, 1, 0, 0)
         phi = K.pool2_fwd(phi_f, 1)                                               # [B, c8, H/2, W/2]  keys  [M][c8]
         g = K.pool2_fwd(g_f, 1)                                                   # [B, c2, H/2, W/2]  values [M][c2]
-        if FUSED_SOFTMAX and M % 64 == 0:
+        if M % 64 == 0:
             # the score GEMM runs twice (K = C/8 is tiny): a statistics pass that stores nothing, then the pass whose epilogue
             # writes P = softmax(theta . phi^T) directly -- the score matrix S never exists in memory
             S, stats = K.conv_fprop(theta, phi, M, 1, 1, 0, 0, w_mode=1, sm_mode=1)
@@ -906,7 +902,7 @@ class SelfAttentionFn(TFunction):
         G_o = K.conv_wgrad(o, dt, 1, 1, 0, 0)
         # o = P . g   ->  dP = do . g^T (keys as output channels), dg = P^T . do (per image)
         dg_pool = K.conv_wgrad(do, P, 1, 1, 0, 0, per_image=True)                 # [B][M][1][c2] fp32
-        if FUSED_SOFTMAX and M % 64 == 0:
+        if M % 64 == 0:
             # dS = P * (dP - delta) in the epilogue of the dP GEMM, delta = rowsum(dP * P) = rowsum(do * o): dP never exists
             dS = K.conv_fprop(do, g, M, 1, 1, 0, 0, w_mode=1, sm_mode=3, sm_delta=K.rowdot(do, o), sm_p=P)
         else:

@@ -5,15 +5,13 @@ Activation convention: a torch tensor of logical shape [B, C, H, W], dtype bfloa
 current CUDA stream of the tensor's device.
 """
 import ctypes
-import os
 
 import torch
 
 from . import _lib as L
 
-# ReLU masks of the discriminators travel to the backward as bit planes (1/16 of the bf16 bytes); SGB_RELU_BITS=0 reads the
-# stored activations instead (A/B switch, read once).
-RELU_BITS = os.environ.get("SGB_RELU_BITS", "1") != "0"
+# ReLU masks of the discriminators travel to the backward as bit planes (1/16 of the bf16 bytes) wherever the layer allows
+# them (conv_fprop want_relu_bits); BITS_STATS counts the planes written and consumed.
 BITS_STATS = {"written": 0, "used": 0}
 
 bf16 = torch.bfloat16
@@ -98,7 +96,7 @@ def conv_fprop(x, w, Cout, KH, KW, pad_h, pad_w, bias=None, residual=None, res_u
         d.mask, d.mask_cstride = mask.data_ptr(), geom(mask)[4]
     d.relu = 1 if relu else 0
     bits = None
-    if want_relu_bits and relu and RELU_BITS and Cout % 64 == 0 and stride == 1 and out.dtype == bf16 and ycs % 8 == 0:
+    if want_relu_bits and relu and Cout % 64 == 0 and stride == 1 and out.dtype == bf16 and ycs % 8 == 0:
         bits = torch.empty((B, H, W, Cout // 8), device=x.device, dtype=torch.uint8)
         d.relu_bits = bits.data_ptr()
         out._sgb_relu_bits = bits

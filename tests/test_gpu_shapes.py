@@ -461,8 +461,7 @@ def test_pool2_bwd_with_bit_planes_and_d_block_uses_them():
     lab = torch.randint(0, 5, (4,), generator=g).to(dev)
     K.BITS_STATS.update(written=0, used=0)
     D(img, lab)["adv_output"].sum().backward()
-    if K.RELU_BITS:
-        assert K.BITS_STATS["written"] > 0 and K.BITS_STATS["used"] >= K.BITS_STATS["written"] - 1, K.BITS_STATS   # (the head reads the last tensor itself)
+    assert K.BITS_STATS["written"] > 0 and K.BITS_STATS["used"] >= K.BITS_STATS["written"] - 1, K.BITS_STATS   # (the head reads the last tensor itself)
 
 
 @pytest.mark.parametrize("B,S,c8,c2", [(2, 64, 64, 256), (3, 16, 48, 192), (1, 32, 16, 64)])
